@@ -6,9 +6,11 @@ reference's test_sr.py:145-197) over one batch of synthetic 32x512 LR text lines
 (BASELINE.json configs[1]; --lines sets lines per GPU per step).  One process per GPU; lines are independent
 (test_sr.py:77) so ranks shard lines with no data-path collective ("weak" scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--lines L] [--chars C]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--lines L] [--chars C] [--dump-outputs DIR]
 
-Prints ONE JSON line on rank 0.  See DESIGN.md "Measurement" for how every field is produced.
+Prints ONE JSON line on rank 0.  See DESIGN.md "Measurement" for how every field is produced.  --dump-outputs DIR writes
+rank 0's SR images of the last timed step as DIR/sr.npy (float32): inputs and weights are seeded and do not depend on the
+host, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -174,7 +176,6 @@ def run_reference_arm(args):
         return
     import torch
     chars, lines = args.chars, args.lines
-    budget_s = 150.0
     warm = max(1, args.warmup)
     t_first, threads = cpu_line_seconds(chars, 1)                      # first warm-up step (also sizes the run)
     per_step = max(t_first, 1e-3) * lines
@@ -182,7 +183,7 @@ def run_reference_arm(args):
     for _ in range(warm - 1):
         for _ in range(lines):
             cpu_line_seconds(chars, 1)
-    steps = max(1, min(args.steps, int(budget_s // per_step)))
+    steps = args.steps
     times = []
     for _ in range(steps):
         t = 0.0
@@ -261,7 +262,7 @@ def run_ours(args):
         barrier()
         ev0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         ev1.record()
         torch.cuda.synchronize()
         ms = ev0.elapsed_time(ev1)
@@ -270,7 +271,7 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
         barrier()
-        return ms
+        return ms, out
 
     with torch.no_grad():
         for _ in range(max(args.warmup, 3)):
@@ -285,8 +286,10 @@ def run_ours(args):
         sampler = ClockSampler(local)
         sampler.start()
         l0 = ops.LAUNCHES
-        ms_total = timed(lambda: step(lq_dev, locs_dev), args.steps)
+        ms_total, out = timed(lambda: step(lq_dev, locs_dev), args.steps)
         launches = (ops.LAUNCHES - l0) // args.steps
+        eager_sr = out.cpu() if args.dump_outputs else None
+        graph_sr = None
         # the same step recorded once into a CUDA graph and replayed (SURVEY 8f n1): identical kernels and results, no Python
         # between launches, label/window checks on the device.  Used for `value` when capture works and replays bit-exactly.
         graph_info, g = None, None
@@ -306,7 +309,9 @@ def run_ours(args):
             if ok.item() > 0.5:
                 for _ in range(2):
                     g.replay()
-                graph_info["ms_per_step"] = timed(g.replay, args.steps) / args.steps
+                ms_graph, out = timed(g.replay, args.steps)
+                graph_info["ms_per_step"] = ms_graph / args.steps
+                graph_sr = out.cpu() if args.dump_outputs else None     # a static buffer: later replays overwrite it
             elif g is not None:
                 graph_info["skipped"] = "another rank could not capture" if graph_info["bit_identical_to_eager"] else "replay differs from eager"
 
@@ -323,7 +328,7 @@ def run_ours(args):
             torch.cuda.current_stream().synchronize()
 
         e2e_step()
-        ms_e2e = timed(e2e_step, args.steps)
+        ms_e2e, _ = timed(e2e_step, args.steps)
 
         roof = modconv_roofline(nets["tspgan"], chars, dev) if rank == 0 else None
         collective = None
@@ -368,6 +373,8 @@ def run_ours(args):
     e2e_value = total_chars / (ms_e2e / args.steps / 1e3)
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, sr=graph_sr if use_graph else eager_sr)
         cpu = None
         if world == 1 and not args.no_cpu_baseline:
             t, threads = cpu_line_seconds(chars, 1)
@@ -401,6 +408,22 @@ def run_ours(args):
         print(json.dumps(rec), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, **arrays):
+    """Writes each array as directory/<name>.npy in float32.  An array larger than DUMP_BYTES / len(arrays) is replaced by a
+    fixed, seeded sample of its flattened elements (same indices on every run of the same shape), in index order."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    budget = (DUMP_BYTES // len(arrays) - 4096) // 4          # elements per file, leaving room for the .npy header
+    for name, t in arrays.items():
+        a = t.float().numpy()
+        if a.size > budget:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, budget, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def collective_record(nets, world, rank, dev, args):
@@ -646,7 +669,14 @@ def main():
     ap.add_argument("--no-collective", action="store_true", help="skip the character-sharded configs[2]/[3] sub-records")
     ap.add_argument("--no-graph", action="store_true", help="skip the CUDA-graph replay measurement (value = eager module calls)")
     ap.add_argument("--profile", action="store_true", help="run one step inside cudaProfilerStart/Stop and exit (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the SR images of rank 0's last timed step as DIR/sr.npy (float32, "
+                         "lines x 3 x 128 x 2048; a seeded sample of its values when that exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -176,9 +176,14 @@ def make_tspsr_sd(seed=3456, power_iters=30):
         u = F.normalize(r.randn(cout), dim=0, eps=1e-12)
         v = F.normalize(r.randn(fan_in), dim=0, eps=1e-12)
         wm = w.flatten(1)
-        for _ in range(power_iters):
-            v = F.normalize(torch.mv(wm.t(), u), dim=0, eps=1e-12)
-            u = F.normalize(torch.mv(wm, v), dim=0, eps=1e-12)
+        threads = torch.get_num_threads()
+        torch.set_num_threads(1)        # torch.mv splits its sums by thread count: one thread gives the same u, v on every host
+        try:
+            for _ in range(power_iters):
+                v = F.normalize(torch.mv(wm.t(), u), dim=0, eps=1e-12)
+                u = F.normalize(torch.mv(wm, v), dim=0, eps=1e-12)
+        finally:
+            torch.set_num_threads(threads)
         sd[p + ".weight_u"] = u
         sd[p + ".weight_v"] = v
 

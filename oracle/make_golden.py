@@ -10,6 +10,7 @@ restatement in oracle/restate.py against them on any machine, and the GPU
 parity tests check the CUDA path against them on the B200 box, where
 /root/reference does not exist.  TEST INFRASTRUCTURE ONLY.
 """
+import contextlib
 import hashlib
 import os
 
@@ -22,6 +23,8 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file
 
 # strides chosen co-prime with the tensor extents so samples hit all channels/rows/cols
 STRIDES = dict(logits=397, locs=1, w=1, image=251, fea64=4099, fea32=2053, sr=1021)
+# denser samples (~15k values per output) for the module-level pin
+MODULE_STRIDES = dict(logits=31, locs=1, w=1, image=7, fea64=127, fea32=67, sr=53)
 
 
 def sample(t, stride):
@@ -62,14 +65,53 @@ def run_reference(models, inp):
                 fea32=torch.cat(p32), sr=sr)
 
 
+# CPU threads the golden fixtures were generated with.  The CPU convolutions split their sums by thread count, so the
+# exact comparisons with them run with the same count whatever the host has.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
+
+
+def modules_case():
+    """Inputs of the module-level pin (tests/test_oracle.py::test_oracle_is_bit_identical_to_reference_modules)."""
+    return synth.make_lq(1, 5), synth.make_labels(2, 9), synth.make_locs(1, 2, ragged=True, seed=3)
+
+
+def write_modules_golden():
+    """tests/golden/modules.npz: samples of every output of the three reference modules for modules_case(), with the
+    reference's own w feeding TSPGAN and its own priors feeding TSPSRNet; w and the encoder locations are stored whole."""
+    sds = synth.make_checkpoints(0)
+    with golden_threads():
+        lq, labels, locs = modules_case()
+        ref = ref_harness.build_reference_models(sds)
+        with torch.no_grad():
+            rl, rlo, rw = ref["encoder"](lq)
+            ri, r64, r32 = ref["tspgan"](styles=rw.repeat(2, 1), labels=labels, noise=None)
+            rs = ref["sr"](lq, [r64], [r32], locs)
+    out = dict(logits=rl, locs=rlo, w=rw, image=ri, fea64=r64, fea32=r32, sr=rs)
+    rec = {k: sample(v, MODULE_STRIDES[k]) for k, v in out.items()}
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "modules.npz"), **rec)
+    print("modules", {k: v.shape for k, v in rec.items()})
+
+
 def main():
     os.makedirs(GOLDEN_DIR, exist_ok=True)
+    write_modules_golden()
     sds = synth.make_checkpoints(0)
     models = ref_harness.build_reference_models(sds)   # strict=True load == key/shape contract
     meta = {k: sd_digest(v) for k, v in sds.items()}
     for name in ("config2", "ragged"):
         inp = case_inputs(name)
-        out = run_reference(models, inp)
+        with golden_threads():
+            out = run_reference(models, inp)
         rec = dict(
             logits=sample(out["logits"], STRIDES["logits"]), locs=sample(out["enc_locs"], 1), w=sample(out["w"], 1),
             image=sample(out["image"], STRIDES["image"]), fea64=sample(out["fea64"], STRIDES["fea64"]),

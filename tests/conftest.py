@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with `-m gpu`)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: runs the reference's own scripts from oracle/_ref/ (staged by build() where the reference tree is readable)")
 
 
 def pytest_collection_modifyitems(config, items):

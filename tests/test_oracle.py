@@ -1,5 +1,5 @@
 """CPU tests: the oracle restatement against the golden fixtures made from the UNMODIFIED reference
-modules (tests/golden, oracle/make_golden.py), and against the reference itself when its tree is present."""
+modules (tests/golden, oracle/make_golden.py)."""
 import os
 
 import numpy as np
@@ -22,11 +22,11 @@ def test_checkpoint_keys_and_digests(checkpoints):
 def test_oracle_matches_reference_golden_ragged(checkpoints):
     """Small case (5 chars, 2 lines): restate.py vs samples of the reference modules' outputs."""
     from oracle import restate
-    from oracle.make_golden import STRIDES, case_inputs
+    from oracle.make_golden import STRIDES, case_inputs, golden_threads
     g = np.load(os.path.join(GOLDEN, "ragged.npz"))
     inp = case_inputs("ragged")
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
-    out = restate.full_line(checkpoints, inp["lq"], inp["labels"], inp["locs"])
+    with golden_threads():
+        out = restate.full_line(checkpoints, inp["lq"], inp["labels"], inp["locs"])
     samp = lambda t, k: t.reshape(-1)[::STRIDES[k]].numpy()
     errs = dict(
         logits=np.abs(samp(out["logits"], "logits") - g["logits"]).max(), w=np.abs(samp(out["w"], "w") - g["w"]).max(),
@@ -62,20 +62,18 @@ def test_clear_labels_ctc_dedup():
     assert restate.clear_labels(logits) == [5, 5, 9]
 
 
-@pytest.mark.reference
 def test_oracle_is_bit_identical_to_reference_modules(checkpoints):
-    from oracle import ref_harness, restate, synth
-    if not ref_harness.available():
-        pytest.skip("reference tree not present (GPU box)")
-    ref = ref_harness.build_reference_models(checkpoints)      # strict=True load of the synthetic checkpoints
-    lq = synth.make_lq(1, 5)
-    labels, locs = synth.make_labels(2, 9), synth.make_locs(1, 2, ragged=True, seed=3)
-    with torch.no_grad():
-        rl, rlo, rw = ref["encoder"](lq)
-        ri, r64, r32 = ref["tspgan"](styles=rw.repeat(2, 1), labels=labels, noise=None)
-        rs = ref["sr"](lq, [r64], [r32], locs)
-    ol, olo, ow = restate.encoder_forward(checkpoints["encoder"], lq)
-    oi, o64, o32 = restate.tspgan_forward(checkpoints["tspgan"], rw.repeat(2, 1), labels)
-    os_ = restate.tspsr_forward(checkpoints["sr"], lq, [r64], [r32], locs)
-    for a, b in ((rl, ol), (rlo, olo), (rw, ow), (ri, oi), (r64, o64), (r32, o32), (rs, os_)):
-        assert (a - b).abs().max().item() <= 1e-6
+    """restate.py vs the outputs of the unmodified reference modules (tests/golden/modules.npz, oracle/make_golden.py), with
+    the thread count they were generated with.  TSPGAN takes the reference's stored w; TSPSRNet takes restate's own priors,
+    which equal the reference's within the same bound."""
+    from oracle import restate
+    from oracle.make_golden import MODULE_STRIDES, golden_threads, modules_case, sample
+    g = np.load(os.path.join(GOLDEN, "modules.npz"))
+    with golden_threads(), torch.no_grad():
+        lq, labels, locs = modules_case()
+        ol, olo, ow = restate.encoder_forward(checkpoints["encoder"], lq)
+        oi, o64, o32 = restate.tspgan_forward(checkpoints["tspgan"], torch.from_numpy(g["w"]).reshape(1, -1).repeat(2, 1), labels)
+        os_ = restate.tspsr_forward(checkpoints["sr"], lq, [o64], [o32], locs)
+    out = dict(logits=ol, locs=olo, w=ow, image=oi, fea64=o64, fea32=o32, sr=os_)
+    for k, t in out.items():
+        assert np.abs(sample(t, MODULE_STRIDES[k]) - g[k]).max() <= 1e-6, k

@@ -74,15 +74,17 @@ def test_oracle_reproduces_the_reference_script_png_row(checkpoints):
     import torch
     from marconet_b200 import pipeline
     from oracle import image_ops, restate
+    from oracle.make_golden import golden_threads
     g = np.load(os.path.join(os.path.dirname(GOLDEN), "script_sr_row.npz"))
     img, boxes, labels, stride = g["image_rgb"], g["boxes"], g["labels"], int(g["stride"])
     lq, lq_w = image_ops.preprocess_lq(img)
     assert lq_w == 256
     lq_t = torch.from_numpy(lq)
     locs = pipeline.boxes_to_locs(boxes.tolist(), img.shape[0], 512)
-    _, _, w = restate.encoder_forward(checkpoints["encoder"], lq_t)
     lab = torch.from_numpy(labels).reshape(-1, 1)
-    _, f64, f32_ = restate.tspgan_forward(checkpoints["tspgan"], w[:1].repeat(lab.shape[0], 1), lab)
-    sr = restate.tspsr_forward(checkpoints["sr"], lq_t, [f64], [f32_], locs)
+    with golden_threads():
+        _, _, w = restate.encoder_forward(checkpoints["encoder"], lq_t)
+        _, f64, f32_ = restate.tspgan_forward(checkpoints["tspgan"], w[:1].repeat(lab.shape[0], 1), lab)
+        sr = restate.tspsr_forward(checkpoints["sr"], lq_t, [f64], [f32_], locs)
     row = image_ops.postprocess_sr(sr.numpy())[0, :, :1024]
     assert np.array_equal(row[::stride, ::stride], g["sr_row"])
