@@ -247,6 +247,20 @@ int mn_window_scatter(const float* feat, int feat_cs, const float* scale, const 
 int mn_char_windows(const float* locs, int locs_stride, const int32_t* line_first, int B, int max_chars, int W, int half,
                     mn_window* win, int32_t* valid, int32_t* owner, int32_t* err, void* stream);
 
+/* Style per character of a line wider than the encoder's input (pipeline.restore_wide_image, DESIGN "Wide lines").  The
+ * encoder (TextViT: 64 tokens, LayerNorm(64) + Linear(64->16) over the token axis, models/textvit_arch.py) only takes 512
+ * columns, so line b of a W-wide canvas is encoded as `segs` segments of seg_w columns, w[b*segs + s][0..dim) (row stride
+ * w_stride).  Character c of line b (characters line_first[b] .. line_first[b+1], device int32[B+1]) gets
+ *   center = (int)(locs[b*locs_stride + 2c] * W)     (fp32 multiply, truncation: the 32-level window centre,
+ *                                                      models/networks.py:426, same arithmetic as mn_char_windows)
+ *   seg    = clamp(floor(center / seg_w), 0, segs-1)
+ *   styles[i*styles_stride + k] = w[(b*segs + seg)*w_stride + k],  seg_out[i] = seg  (seg_out may be NULL),  i = line_first[b]+c.
+ * With segs == 1 every character gets its line's w, which is what test_sr.py:147-181 feeds TSPGAN (w0.repeat(n, 1)).
+ * max_chars >= the longest line. */
+int mn_char_segment_styles(const float* w, int w_stride, const float* locs, int locs_stride, const int32_t* line_first,
+                           int B, int max_chars, int W, int seg_w, int segs, int dim, float* styles, int styles_stride,
+                           int32_t* seg_out, void* stream);
+
 /* The reference module's standalone helper functions on NCHW-contiguous tensors (rows = B*C, len = H*W); the hot path uses
  * the fused NHWC kernels above.
  *   mn_swish         x * sigmoid(x)                                                models/networks.py:492-493

@@ -66,6 +66,8 @@ SYMBOLS = {
     "mn_set_pdl": (c_int, [c_int]),
     "mn_check_labels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "mn_char_windows": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mn_char_segment_styles": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
+                                       c_void_p, c_void_p]),
     "mn_demod": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "mn_demod_batched": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
     "mn_resample_modulate": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),

@@ -320,6 +320,26 @@ __global__ void char_windows_kernel(const float* __restrict__ locs, int locs_str
     }
 }
 
+// ---------------------------------------------------------------- style per character of a wide line
+// A line wider than the encoder's 512 columns is encoded as `segs` segments of seg_w columns (one style row each).  Character c
+// of line b takes the style of the segment holding its centre, computed with the 32-level window centre's arithmetic
+// (networks.py:426: fp32 multiply, truncation toward zero) and clamped into [0, segs).  One CTA per character.
+__global__ void char_segment_styles_kernel(const float* __restrict__ w, int w_stride, const float* __restrict__ locs, int locs_stride,
+                                           const int32_t* __restrict__ line_first, int W, int seg_w, int segs, int dim,
+                                           float* __restrict__ styles, int styles_stride, int32_t* __restrict__ seg_out) {
+    mn_pdl_prologue();
+    const int b = blockIdx.y, c = blockIdx.x;
+    const int first = line_first[b];
+    if (c >= line_first[b + 1] - first) return;
+    const int center = __float2int_rz(__fmul_rn(locs[(size_t)b * locs_stride + 2 * c], (float)W));
+    int seg = center < 0 ? 0 : center / seg_w;
+    if (seg > segs - 1) seg = segs - 1;
+    const float* src = w + (size_t)(b * segs + seg) * w_stride;
+    float* dst = styles + (size_t)(first + c) * styles_stride;
+    for (int k = threadIdx.x; k < dim; k += blockDim.x) dst[k] = src[k];
+    if (seg_out && threadIdx.x == 0) seg_out[first + c] = seg;
+}
+
 // ---------------------------------------------------------------- standalone helper functions of the reference module
 // swish (networks.py:492-493), calc_mean_std_4D (:518-525), adaptive_instance_normalization (:528-533) on NCHW-contiguous
 // tensors, rows = B*C, len = H*W.  The hot path uses the fused NHWC kernels above; these keep the reference's module-level
@@ -499,6 +519,19 @@ extern "C" int mn_char_windows(const float* locs, int locs_stride, const int32_t
     MN_REQUIRE(B > 0 && W > 0 && half > 0 && max_chars >= 0 && max_chars <= 4096, "mn_char_windows: bad dims");
     MN_CUDA_CHECK((mn_launch(char_windows_kernel, dim3(B), dim3(256), (size_t)max_chars * 2 * sizeof(int32_t), (cudaStream_t)stream,
                              locs, locs_stride, line_first, W, half, win, valid, owner, err)));
+    MN_LAUNCH_CHECK();
+    return MN_OK;
+}
+
+extern "C" int mn_char_segment_styles(const float* w, int w_stride, const float* locs, int locs_stride, const int32_t* line_first,
+                                      int B, int max_chars, int W, int seg_w, int segs, int dim, float* styles, int styles_stride,
+                                      int32_t* seg_out, void* stream) {
+    MN_REQUIRE(w && locs && line_first && styles, "mn_char_segment_styles: null pointer");
+    MN_REQUIRE(B > 0 && W > 0 && seg_w > 0 && segs > 0 && dim > 0 && max_chars >= 0 && max_chars <= 65535 && B <= 65535 &&
+               w_stride >= dim && styles_stride >= dim && (int64_t)B * segs < (1ll << 31), "mn_char_segment_styles: bad dims");
+    if (max_chars == 0) return MN_OK;
+    MN_CUDA_CHECK((mn_launch(char_segment_styles_kernel, dim3(max_chars, B), dim3(128), 0, (cudaStream_t)stream,
+                             w, w_stride, locs, locs_stride, line_first, W, seg_w, segs, dim, styles, styles_stride, seg_out)));
     MN_LAUNCH_CHECK();
     return MN_OK;
 }

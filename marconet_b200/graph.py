@@ -7,6 +7,8 @@ CUDA graph and replayed: no Python between the ~220 launches, no host round trip
 as device kernels inside ``ops.deferred_checks``; their error bits are read back together with the result).
 
 The flow is the one of test_sr.py: labels and boxes come from the caller (OCR / detector), the style ``w`` from the encoder.
+Lines wider than 512 columns (``width`` a multiple of 64) follow pipeline.restore_wide_image: the encoder runs on the 512-column
+segments of every line and each character takes the style of the segment that holds its centre (mn_char_segment_styles).
 """
 import torch
 
@@ -17,10 +19,12 @@ class GraphedLines:
     """encoder -> TSPGAN -> TSPSRNet for ``lines`` LR lines of ``chars`` characters each, as one CUDA graph.
 
     >>> g = GraphedLines(encoder, tspgan, sr, lines=1, chars=16)
-    >>> out = g(lq, labels, locs)      # lq [lines,3,32,512] fp32, labels int64 [lines*chars,1], locs fp32 [lines,2*chars]
+    >>> out = g(lq, labels, locs)      # lq [lines,3,32,width] fp32, labels int64 [lines*chars,1], locs fp32 [lines,2*chars]
     >>> g.check()                      # raises what the eager modules would have raised (reads 4 bytes back)
 
-    ``out`` (and everything in ``g.outputs``) is a static buffer that the next call overwrites."""
+    ``out`` (and everything in ``g.outputs``) is a static buffer that the next call overwrites.  ``width`` is 512 (the reference
+    canvas) or any multiple of 64 above it up to pipeline.WIDE_MAX_WIDTH (wide lines: ``lq`` is the canvas restore_wide_image
+    builds, locs are in units of ``width``, and ``outputs`` also holds ``seg``, the encoder segment of every character)."""
 
     def __init__(self, encoder, tspgan, sr, lines=1, chars=16, height=32, width=512, device=None, warmup=2, overlap_trunk=True):
         if device is None:
@@ -30,9 +34,21 @@ class GraphedLines:
             raise RuntimeError("GraphedLines: the modules must live on a CUDA (sm_100a) device; there is no CPU fallback")
         if lines < 1 or chars < 1:
             raise RuntimeError("GraphedLines: lines and chars must be positive")
+        from .pipeline import WIDE_ALIGN, WIDE_MAX_WIDTH, WIDE_SEGMENT
+        if width < WIDE_SEGMENT or width % WIDE_ALIGN or width > WIDE_MAX_WIDTH:
+            raise RuntimeError(f"GraphedLines: width {width} must be a multiple of {WIDE_ALIGN} in [{WIDE_SEGMENT}, {WIDE_MAX_WIDTH}]")
         self.encoder, self.tspgan, self.sr = encoder, tspgan, sr
-        self.lines, self.chars, self.device = lines, chars, device
-        self.lq = torch.zeros((lines, 3, height, width), dtype=torch.float32, device=device)
+        self.lines, self.chars, self.device, self.width = lines, chars, device, width
+        self.segments = -(-width // WIDE_SEGMENT)
+        if self.segments == 1:
+            self._canvas = None
+            self.lq = torch.zeros((lines, 3, height, width), dtype=torch.float32, device=device)
+        else:
+            # encoder input: the lines extended to whole 512-column segments with the canvas padding (-1 = the zero byte
+            # normalised); lq is a view of its first ``width`` columns, so load() writes straight into it
+            self._canvas = torch.full((lines, 3, height, self.segments * WIDE_SEGMENT), -1.0, dtype=torch.float32, device=device)
+            self.lq = self._canvas[..., :width]
+            self._line_first = torch.arange(0, (lines + 1) * chars, chars, dtype=torch.int32).to(device)
         self.labels = torch.zeros((lines * chars, 1), dtype=torch.int64, device=device)
         # default boxes: evenly spaced, so that warm-up and capture never see an empty window
         locs = torch.zeros((lines, 2 * chars), dtype=torch.float32)
@@ -77,8 +93,17 @@ class GraphedLines:
                     trunk_done.record(branch)
             # the encoder's classification / box branches and the generator's ToRGB chain also go to the second stream: the
             # generator only waits for w, the SR decoder only for the feature taps and the trunk
-            logits, locs_lr, w = self.encoder(self.lq, _branch=(branch, self._trunk_ws) if branch is not None else None)
-            image, f64, f32_ = self.tspgan(styles=w.repeat_interleave(self.chars, dim=0), labels=self.labels, noise=None, _branch=branch)
+            enc_branch = (branch, self._trunk_ws) if branch is not None else None
+            seg = None
+            if self._canvas is None:      # the reference canvas: one segment, every character of line b gets w[b]
+                logits, locs_lr, w = self.encoder(self.lq, _branch=enc_branch)
+                styles = w.repeat_interleave(self.chars, dim=0)
+            else:
+                from .pipeline import WIDE_SEGMENT, _encoder_segments
+                logits, locs_lr, w = self.encoder(_encoder_segments(self._canvas, self.segments), _branch=enc_branch)
+                styles, seg = ops.char_segment_styles(w, self.locs, self._line_first, [self.chars] * self.lines, self.width,
+                                                      self.segments, WIDE_SEGMENT)
+            image, f64, f32_ = self.tspgan(styles=styles, labels=self.labels, noise=None, _branch=branch)
             n = self.chars
             p64 = [f64[b * n:(b + 1) * n] for b in range(self.lines)]
             p32 = [f32_[b * n:(b + 1) * n] for b in range(self.lines)]
@@ -88,7 +113,10 @@ class GraphedLines:
             out = self.sr(self.lq, p64, p32, self.locs, _trunk=trunk)
             if branch is not None:
                 main.wait_stream(branch)                       # joins logits / locs and the prior image
-        return dict(sr=out, prior=image, fea64=f64, fea32=f32_, logits=logits, locs_lr=locs_lr, w=w)
+        outs = dict(sr=out, prior=image, fea64=f64, fea32=f32_, logits=logits, locs_lr=locs_lr, w=w)
+        if seg is not None:
+            outs["seg"] = seg
+        return outs
 
     def load(self, lq=None, labels=None, locs=None):
         """Copy new inputs (host or device tensors) into the static buffers on the current stream."""

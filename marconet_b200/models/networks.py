@@ -765,17 +765,34 @@ class TSPSRNet(_PackedModule):
         s32 = _two(pk["conv_body_32"], cat32)
         return s32
 
+    @staticmethod
+    def _check_geometry(lq, priors32=()):
+        """Shapes the reference module rejects, raised before anything is launched: the two stride-2 convs and the two x2
+        up-samplings of the trunk only line up (torch.cat at networks.py:415-416) when H and W are multiples of 4, and the 32-px
+        priors are concatenated with H-row windows of the 32-level map (networks.py:442-445), so H must be 32 when any line has
+        characters.  (Without the first check, W = 2 mod 4 would make the up-sampled 8-row map one column wider than its slot.)"""
+        if lq.dim() != 4:
+            raise RuntimeError(f"TSPSRNet: lq must be [B, 3, H, W], got {tuple(lq.shape)}")
+        h, w = int(lq.shape[2]), int(lq.shape[3])
+        if h % 4 or w % 4:
+            raise RuntimeError(f"TSPSRNet: LR line of {h}x{w}; height and width must be multiples of 4 (the reference fails in "
+                               f"torch.cat at networks.py:415-416)")
+        if h != 32 and any(int(p.shape[0]) > 0 for p in priors32):
+            raise RuntimeError(f"TSPSRNet: LR line height {h} with characters; the 32x32 priors need height 32 (networks.py:442-445)")
+
     @torch.no_grad()
     def trunk(self, lq):
         """Public handle on the LR trunk so that a pipeline can launch it early, on a second stream, while the encoder and the
         prior generator run (it needs only the LR line): pass the result to forward(..., _trunk=...)."""
         self._need_cuda(lq, "TSPSRNet")
+        self._check_geometry(lq)
         with ops.on_device(lq):
             return self._trunk(self._get_packed(lq.device), lq)
 
     @torch.no_grad()
     def forward(self, lq, priors64, priors32, locs, _trunk=None):
         self._need_cuda(lq, "TSPSRNet")
+        self._check_geometry(lq, priors32)
         with ops.on_device(lq):
             ent = self._forward_graphed(lq, priors64, priors32, locs) if _trunk is None else None
             if ent is not None:

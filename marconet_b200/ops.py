@@ -575,6 +575,31 @@ def char_windows(locs_dev, line_first_dev, counts, width, half, flag):
     return win, valid, owner
 
 
+def char_segment_styles(w, locs_dev, line_first_dev, counts, width, segs, seg_w=512):
+    """mn_char_segment_styles: style row of every character of B wide lines, taken from the encoder segment that holds the
+    character's 32-level window centre.  ``w``: [B*segs, D] (row b*segs + s = segment s of line b); ``locs_dev``: fp32 [B, >= 2n]
+    on the device; ``line_first_dev``: device int32[B+1] prefix sums of ``counts``.  Returns (styles [Nc, D], seg int32 [Nc])."""
+    global LAUNCHES
+    _require_cuda(w, "w")
+    _require_cuda(locs_dev, "locs")
+    b, nc = len(counts), sum(counts)
+    if w.dim() != 2 or w.stride(1) != 1 or w.shape[0] != b * segs:
+        raise RuntimeError(f"char_segment_styles: w must be [{b * segs}, D] with unit inner stride, got {tuple(w.shape)}")
+    if locs_dev.dim() != 2 or locs_dev.stride(1) != 1 or locs_dev.shape[0] < b or (counts and locs_dev.shape[1] < 2 * max(counts)):
+        raise RuntimeError("char_segment_styles: locs must be fp32 [B, >= 2n] with unit inner stride")
+    if line_first_dev.dtype != torch.int32 or not line_first_dev.is_cuda or line_first_dev.numel() != b + 1:
+        raise RuntimeError("char_segment_styles: line_first must be a device int32[B+1] tensor")
+    styles = torch.empty((nc, w.shape[1]), dtype=torch.float32, device=w.device)
+    seg = torch.empty((nc,), dtype=torch.int32, device=w.device)
+    if nc == 0:
+        return styles, seg
+    _lib.check(_lib.load().mn_char_segment_styles(_ptr(w), w.stride(0), _ptr(locs_dev), locs_dev.stride(0), _ptr(line_first_dev), b,
+                                                  max(counts), width, seg_w, segs, w.shape[1], _ptr(styles), styles.stride(0), _ptr(seg),
+                                                  _stream()), "mn_char_segment_styles")
+    LAUNCHES += 1
+    return styles, seg
+
+
 def select_text(emb, labels_dev, s, n, l):
     """emb: [classes, C]; labels_dev: int64 [n*l] on device; s: [n, C] view (row stride s.stride(0)) or None."""
     global LAUNCHES
@@ -626,7 +651,9 @@ def resample_modulate(x, s=None, up=False, out=None):
     n, h, w, c, x_cs = nhwc_info(x, "x")
     oh, ow = (2 * h, 2 * w) if up else (h, w)
     y = out if out is not None else torch.empty((n, oh, ow, c), dtype=torch.float32, device=x.device)
-    _, _, _, _, y_cs = nhwc_info(y, "out")
+    yn, yh, yw, yc, y_cs = nhwc_info(y, "out")
+    if (yn, yh, yw, yc) != (n, oh, ow, c):
+        raise RuntimeError(f"resample_modulate: out has shape {tuple(y.shape)}, expected {(n, oh, ow, c)}")
     _lib.check(_lib.load().mn_resample_modulate(_ptr(x), x_cs, _ptr(y), y_cs, _ptr(s), 0 if s is None else s.stride(0),
                                                 n, h, w, c, 1 if up else 0, _stream()), "mn_resample_modulate")
     LAUNCHES += 1

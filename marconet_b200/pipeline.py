@@ -6,6 +6,8 @@ boxes converted from the encoder's (left, right) pairs to (centre, half-width) e
 (Train/tspgan/models/tspgan_model.py:331-337).  Integer outputs (labels) are computed on the host, bit-exactly like the
 reference; everything numeric runs through the module API (and therefore through the CUDA kernels).
 """
+import collections
+
 import torch
 
 ALPHABET_SIZE = 6735          # classes [0, 6735) are characters, 6735 is the CTC blank (utils/alphabets.py, test_w.py:38)
@@ -119,6 +121,103 @@ def restore_image(encoder, tspgan, sr, img_u8, labels, boxes):
     show_w = ops.round_half_even(img.shape[1] * (128 / h))    # ShowLQ = cv2.resize(img, fx=128/h, ...) (test_sr.py:98)
     sr_u8 = ops.postprocess_sr(out)[0, :, :show_w]            # ShowSR = sr[:, :ShowLQ.shape[1]] (test_sr.py:201)
     return dict(sr_u8=sr_u8, sr=out, lq=lq, lq_width=lq_w, prior=img_prior, locs=locs)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Lines wider than 512 LR columns (DESIGN.md "Wide lines").  The reference script pastes the 32-px-high line onto a 32x512 canvas
+# and skips anything wider (test_sr.py:104-110).  Only the encoder is fixed at 512 columns (TextViT: 64 tokens); TSPSRNet is
+# width-generic (its window integers use the map's own width, networks.py:426,435,460,469).  So the line is restored in ONE
+# SR pass on a wider canvas, and the encoder runs on 512-column segments of it, each character taking the style of the
+# segment that holds its centre.
+# ---------------------------------------------------------------------------------------------------------------------
+WIDE_SEGMENT = 512          # encoder input width (TextViT: 64 tokens of 8x8 patches over an 8x512 feature map)
+WIDE_ALIGN = 64             # canvas width granularity: W/4 % 16 == 0 keeps every SR layer on the tcgen05 kernel (DESIGN 3.1)
+# Largest canvas every kernel on the path can index: the biggest map is conv_final's up-sampled input, 128 channels at
+# 128 x 4*Wsr pixels, and the elementwise / GroupNorm / conv epilogue kernels index maps with 32-bit element (or 4-element)
+# counts (checked against 2^31 on the host, e.g. mn_resample_modulate, mn_groupnorm_apply, mn_conv2d_nhwc's M); 128*4*Wsr*128
+# < 2^31 gives Wsr < 32768.  The owner tables (B*Wsr int32) and the preprocess canvas (3*32*S*512 floats) are far below it.
+WIDE_MAX_WIDTH = ((2 ** 31 - 1) // (128 * 4 * 128)) // WIDE_ALIGN * WIDE_ALIGN          # 32704
+
+
+# (Wr, Wsr, S, show_w) of one h x w image; compares equal to the plain tuple
+WideGeometry = collections.namedtuple("WideGeometry", "lq_width canvas_width segments show_width")
+
+
+def wide_geometry(h, w):
+    """Canvas of an h x w line image, in Python floats as test_sr.py / cv::resize compute them:
+      Wr     = round_half_even(w * (32/h))           the resized LQ width (cv2.resize with fx = 32/h, test_sr.py:99)
+      Wsr    = max(512, 64 * ceil(Wr / 64))          the SR canvas, zero-padded on the right like the script's 512 canvas
+      S      = ceil(Wsr / 512)                        encoder segments: canvas columns [512 s, 512 s + 512), zero-extended
+      show_w = round_half_even(w * (128/h))          ShowLQ's width (test_sr.py:98); the output is sr[:, :show_w]
+    Lines with Wr <= 512 get Wsr = 512, S = 1: exactly the script's canvas."""
+    from .ops import round_half_even
+    h, w = int(h), int(w)
+    if h <= 0 or w <= 0:
+        raise ValueError(f"empty image ({h} x {w})")
+    wr = round_half_even(w * (32 / h))
+    wsr = max(WIDE_SEGMENT, WIDE_ALIGN * (-(-wr // WIDE_ALIGN)))
+    return WideGeometry(wr, wsr, -(-wsr // WIDE_SEGMENT), round_half_even(w * (128 / h)))
+
+
+def _encoder_segments(canvas, segs):
+    """[B, 3, 32, segs*512] canvas -> [B*segs, 3, 32, 512] (a strided view when B == 1; the encoder's NCHW->NHWC copy reads it)."""
+    b, c, hh, _ = canvas.shape
+    v = canvas.reshape(b, c, hh, segs, WIDE_SEGMENT).permute(0, 3, 1, 2, 4)
+    return v[0] if b == 1 else v.reshape(b * segs, c, hh, WIDE_SEGMENT)
+
+
+@torch.no_grad()
+def wide_lines_forward(encoder, tspgan, sr, canvas, labels, locs, width, chars):
+    """The wide-line data flow on preprocessed canvases: ``canvas`` fp32 [B, 3, 32, S*512] on the device (padding = -1, the
+    normalised zero byte), ``labels`` int64 [B*chars, 1], ``locs`` fp32 device [B, 2*chars] in units of ``width`` (= Wsr, a
+    multiple of 64, at least 512).  encoder on the B*S segments -> mn_char_segment_styles -> one TSPGAN call -> one TSPSRNet call
+    on canvas[..., :width].  Returns dict(sr, prior, fea64, fea32, w, seg)."""
+    from . import ops
+    b = canvas.shape[0]
+    segs = canvas.shape[-1] // WIDE_SEGMENT
+    _, _, w = encoder(_encoder_segments(canvas, segs))
+    first = torch.arange(0, (b + 1) * chars, chars, dtype=torch.int32).to(canvas.device, non_blocking=True)
+    styles, seg = ops.char_segment_styles(w, locs, first, [chars] * b, width, segs, WIDE_SEGMENT)
+    image, f64, f32_ = tspgan(styles=styles, labels=labels, noise=None)
+    p64 = [f64[i * chars:(i + 1) * chars] for i in range(b)]
+    p32 = [f32_[i * chars:(i + 1) * chars] for i in range(b)]
+    out = sr(canvas[..., :width], p64, p32, locs)
+    return dict(sr=out, prior=image, fea64=f64, fea32=f32_, w=w, seg=seg)
+
+
+@torch.no_grad()
+def restore_wide_image(encoder, tspgan, sr, img_u8, labels, boxes):
+    """restore_image for a line of any width: uint8 [h, w, 3] image -> the same keys as restore_image plus ``segments`` (S),
+    ``w`` ([S, 512], one style per encoder segment) and ``seg`` (int32 [n], the segment each character's style came from).
+
+    The line is resized to height 32 (Wr columns) and pasted on a Wsr = max(512, 64*ceil(Wr/64)) canvas (wide_geometry); the
+    encoder sees the S = ceil(Wsr/512) segments of it as one batch; character i takes w[seg_i] with seg_i the segment holding its
+    32-level window centre; TSPGAN runs once for all characters and TSPSRNet once on [1, 3, 32, Wsr] -- no seams.  For Wr <= 512
+    every step is restore_image's (same canvas, S = 1, every character gets w[0]), and the results are identical.
+    Raises ValueError before launching anything when there are no labels or the canvas exceeds WIDE_MAX_WIDTH."""
+    from . import ops
+    img = torch.as_tensor(img_u8)
+    if img.dim() != 3:
+        raise ValueError(f"expected a uint8 [h, w, c] image, got shape {tuple(img.shape)}")
+    h, w = int(img.shape[0]), int(img.shape[1])
+    geo = wide_geometry(h, w)
+    if geo.canvas_width > WIDE_MAX_WIDTH:
+        raise ValueError(f"line of {h}x{w} px needs a {geo.canvas_width}-column LR canvas; at most {WIDE_MAX_WIDTH} columns fit the "
+                         f"kernels' 32-bit indexing: crop it into shorter segments")
+    lab = torch.as_tensor(labels, dtype=torch.long).reshape(-1, 1)
+    n = lab.shape[0]
+    if n == 0:
+        raise ValueError("no character labels (test_sr.py:160-162 skips such images)")
+    if len(boxes) < n:
+        raise ValueError(f"{n} labels but only {len(boxes)} boxes")
+    dev = next(encoder.parameters()).device
+    img = img.to(dev, non_blocking=True).contiguous()
+    canvas, lq_w = ops.preprocess_lq(img, out_w=geo.segments * WIDE_SEGMENT)
+    locs = boxes_to_locs(boxes, h, geo.canvas_width).to(dev)
+    out = wide_lines_forward(encoder, tspgan, sr, canvas, lab, locs, geo.canvas_width, n)
+    sr_u8 = ops.postprocess_sr(out["sr"])[0, :, :geo.show_width]      # ShowSR = sr[:, :ShowLQ.shape[1]] (test_sr.py:201)
+    return dict(sr_u8=sr_u8, sr=out["sr"], lq=canvas[..., :geo.canvas_width], lq_width=lq_w, prior=out["prior"], locs=locs,
+                segments=geo.segments, w=out["w"], seg=out["seg"])
 
 
 # ---------------------------------------------------------------------------------------------------------------------
