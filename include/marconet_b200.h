@@ -99,7 +99,7 @@ typedef struct {
     /* tensor-core precisions only: weights pre-split by mn_conv_pack_weights_tc()                */
     const void* w_tc_hi; const void* w_tc_lo;  /* 16-bit [KH*KW][Cout][Cin] (K-major)            */
     const float* w_tc_scale;                   /* the 2-float scale record written by the packer */
-    /* optional input transform fused into the tcgen05 v2 kernel's operand-split stage (mn_conv2d_tc_version() == 2 only):
+    /* optional input transform fused into the tcgen05 kernel's operand-split stage (tensor-core path only):
      *   x' = swish( (x - mean[n,g]) * rstd[n,g] * gamma[c] + beta[c] ),  zero outside the image / beyond valid_w[n]
      * i.e. GroupNorm(32 channels per group) + swish of models/networks.py:508-512 applied while the A operand is built (its own
      * kernel instantiation: four lanes per halo row, constants in registers).  Needs OH*OW >= 128 (one sample per 128-pixel tile);
@@ -122,23 +122,22 @@ typedef struct {
      * memory of PEER GPUs (NVLink-mapped symmetric memory): the epilogue's stores then deliver every character's prior features
      * straight into the buffer of the rank that runs that character's SR decoder, tile by tile, while the MMAs of the next tile run
      * -- the exchange of the character-sharded path (reference consumer: models/networks.py:442-445, 475-478) without a separate
-     * collective.  tcgen05 v2 kernel only, layers whose samples are whole pixel tiles (OH*OW >= 128), no split-K. */
+     * collective.  Tensor-core path only, layers whose samples are whole pixel tiles (OH*OW >= 128), no split-K. */
     float* const* y2_ptrs;
     /* GroupNorm statistics of the OUTPUT accumulated by the epilogue (models/networks.py:508-512: the tensor this convolution writes
      * is normalised next): per (sample, group of 32 output channels) sum and sum of squares of y, fp32 partials per warp and tile
      * added into [N][Cout/32][2] doubles with atomics (the caller zeroes the buffer; columns beyond valid_w contribute 0).
-     * tcgen05 v2 kernel, whole-tile samples (OH*OW >= 128), no split-K; finish with mn_groupnorm_finalize. */
+     * Tensor-core path only, whole-tile samples (OH*OW >= 128), no split-K; finish with mn_groupnorm_finalize. */
     double* gn_stats_out;
 } mn_conv_params;
 
 int mn_conv2d_nhwc(const mn_conv_params* p, void* stream);
 /* Bytes of workspace mn_conv2d_nhwc wants for this problem (0 if it will not split). */
 int64_t mn_conv2d_workspace_bytes(const mn_conv_params* p);
-/* 1 if the tcgen05 path can run this geometry (stride 1, 3x3/pad1 or 1x1, Cin%64==0, Cout%64==0,
- * pixel tiles of 128 that tile [N,H,W] exactly); 0 otherwise (mn_last_error() says why). */
+/* 1 if the tcgen05 path can run this geometry (stride 1, 3x3/pad1 or 1x1, Cin%64==0, Cout%64==0, H a multiple of 8 or a
+ * power of two below 8, W a multiple of 128/min(H,8) or a power of two below that, a halo tile of at most 208 rows, 16-byte
+ * aligned operands); 0 otherwise (mn_last_error() says why). */
 int mn_conv2d_tc_supported(const mn_conv_params* p);
-/* 2: the tcgen05 v2 kernel (halo tiles, fused input transforms) runs this problem; 1: only the v1 kernel; 0: neither. */
-int mn_conv2d_tc_version(const mn_conv_params* p);
 /* Split fp32 weights w:[taps*Cin][Cout] (the layout mn_conv2d_nhwc takes) into hi/lo 16-bit planes
  * [taps][Cout][Cin], pre-scaled by a power of two so the lo plane stays in the fp16 normal range.
  * hi, lo: taps*Cin*Cout 16-bit elements each; scale2: 2 floats {abs-max, 2^-S}. */

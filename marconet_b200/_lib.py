@@ -55,7 +55,6 @@ SYMBOLS = {
     "mn_conv2d_nhwc": (c_int, [POINTER(ConvParams), c_void_p]),
     "mn_conv2d_workspace_bytes": (c_int64, [POINTER(ConvParams)]),
     "mn_conv2d_tc_supported": (c_int, [POINTER(ConvParams)]),
-    "mn_conv2d_tc_version": (c_int, [POINTER(ConvParams)]),
     "mn_groupnorm_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
     "mn_groupnorm_finalize": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p]),
     "mn_groupnorm_apply": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,

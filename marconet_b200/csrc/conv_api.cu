@@ -2,13 +2,6 @@
 #include "mn_common.cuh"
 #include "conv_common.cuh"
 
-#include <stdlib.h>
-static bool tc_force_v1() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("MN_TC_V1"); v = (e && e[0] == '1') ? 1 : 0; }
-    return v == 1;
-}
-
 static int make_geom(const mn_conv_params* p, ConvGeom& g) {
     MN_REQUIRE(p != nullptr, "mn_conv2d_nhwc: null params");
     MN_REQUIRE(p->x && p->w && (p->y || p->y2), "mn_conv2d_nhwc: null x/w/y");
@@ -56,26 +49,20 @@ extern "C" int mn_conv2d_nhwc(const mn_conv_params* p, void* stream) {
     int rc = make_geom(p, g);
     if (rc != MN_OK) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const bool v2 = p->precision != MN_PREC_FP32_SIMT && !tc_force_v1() && mn_conv_tc2_supported(g, nullptr);
-    if ((g.y2_ptrs || g.gn_stats_out) && !v2) {
-        mn_set_error("mn_conv2d_nhwc: per-sample output pointers (y2_ptrs) / epilogue GroupNorm statistics (gn_stats_out) exist only in the tcgen05 v2 kernel");
-        return MN_ERR_UNSUPPORTED;
-    }
-    if (g.gn_mr && !v2) {
-        mn_set_error("mn_conv2d_nhwc: the fused GroupNorm input transform exists only in the tcgen05 v2 kernel (check mn_conv2d_tc_version)");
-        return MN_ERR_UNSUPPORTED;
-    }
     switch (p->precision) {
         case MN_PREC_FP32_SIMT:
+            if (g.gn_mr || g.y2_ptrs || g.gn_stats_out) {
+                mn_set_error("mn_conv2d_nhwc: the fused GroupNorm input transform (gn_mean_rstd), per-sample output pointers (y2_ptrs) and "
+                             "epilogue GroupNorm statistics (gn_stats_out) need the tensor-core path");
+                return MN_ERR_UNSUPPORTED;
+            }
             if (mn_conv_small_supported(g)) return mn_conv_small_launch(g, st);
             g.splits = mn_conv_simt_plan_splits(g, p->workspace ? p->workspace_bytes : 0, p->split_k);
             return mn_conv_simt_launch(g, nullptr, st);
         case MN_PREC_F16X3_TC:
         case MN_PREC_BF16X3_TC:
         case MN_PREC_F16X1_TC:
-            if (!tc_force_v1() && mn_conv_tc2_supported(g, nullptr))
-                return mn_conv_tc2_launch(g, p->w_tc_hi, p->w_tc_lo, p->w_tc_scale, p->precision, st);
-            return mn_conv_tc_launch(g, p->w_tc_hi, p->w_tc_lo, p->w_tc_scale, p->precision, st);
+            return mn_conv_tc2_launch(g, p->w_tc_hi, p->w_tc_lo, p->w_tc_scale, p->precision, st);
         default:
             mn_set_error("mn_conv2d_nhwc: unknown precision mode %d", p->precision);
             return MN_ERR_UNSUPPORTED;
@@ -86,14 +73,7 @@ extern "C" int mn_conv2d_tc_supported(const mn_conv_params* p) {
     ConvGeom g;
     if (make_geom(p, g) != MN_OK) return 0;
     const char* why = "";
-    const int ok = (!tc_force_v1() && mn_conv_tc2_supported(g, nullptr)) || mn_conv_tc_supported(g, &why);
+    const int ok = mn_conv_tc2_supported(g, &why);
     if (!ok) mn_set_error("tensor-core path unsupported: %s", why);
     return ok;
-}
-
-extern "C" int mn_conv2d_tc_version(const mn_conv_params* p) {
-    ConvGeom g;
-    if (make_geom(p, g) != MN_OK) return 0;
-    if (!tc_force_v1() && mn_conv_tc2_supported(g, nullptr)) return 2;
-    return mn_conv_tc_supported(g, nullptr) ? 1 : 0;
 }

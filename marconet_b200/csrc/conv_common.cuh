@@ -7,7 +7,7 @@ struct ConvGeom {
     float* y; float* y2;
     const float* bias; const float* out_scale; const float* residual; const float* y2_scale;
     const int32_t* valid_w; float* ws; int64_t ws_bytes;
-    const float2* gn_mr; const float* gn_gamma; const float* gn_beta; int gn_swish;   // fused GroupNorm(+swish) on the input (tc2 only)
+    const float2* gn_mr; const float* gn_gamma; const float* gn_beta; int gn_swish;   // fused GroupNorm(+swish) on the input (tensor-core path only)
     int N, H, W, Cin, x_cs;
     int KH, KW, sh, sw, ph, pw, Cout;
     int OH, OW, y_cs, y2_cs, res_cs, res_bcast, os_stride, y2s_stride;
@@ -15,8 +15,8 @@ struct ConvGeom {
     int M, K;
     int ktiles, ktiles_per_split, splits;
     float x_scale; float* x_absmax; int32_t* range_flag; int32_t range_tag;   // fp16-range management (tensor-core precisions)
-    float* const* y2_ptrs;     // per-sample base pointers of the second output (peer-GPU stores), tcgen05 v2 kernel only
-    double* gn_stats_out;      // [N][Cout/32][2] sum / sum of squares of the output (GroupNorm statistics in the epilogue), v2 only
+    float* const* y2_ptrs;     // per-sample base pointers of the second output (peer-GPU stores), tensor-core path only
+    double* gn_stats_out;      // [N][Cout/32][2] sum / sum of squares of the output (GroupNorm statistics in the epilogue), tensor-core path only
 };
 
 // Range bookkeeping of the operand-split stage: `amax` = bits of the running fmaxf(|x * x_scale|) a thread has seen (fmaxf drops
@@ -145,10 +145,7 @@ int mn_conv_simt_plan_splits(const ConvGeom& g, int64_t ws_bytes, int requested)
 int mn_conv_simt_launch(ConvGeom g, const float* unused, cudaStream_t st);
 int mn_conv_splitk_reduce_launch(const ConvGeom& g, cudaStream_t st);   // sums g.splits partial tiles in g.ws and runs the fused epilogue
 
-// tcgen05 path (conv_tc.cu)
-int mn_conv_tc_supported(const ConvGeom& g, const char** why);
-int mn_conv_tc_launch(const ConvGeom& g, const void* w_hi, const void* w_lo, const float* w_scale, int prec, cudaStream_t st);
-// tcgen05 path v2: halo tiles + weight multicast + persistent CTAs (conv_tc2.cu)
+// tcgen05 path: halo tiles + weight multicast + persistent CTAs (conv_tc2.cu)
 int mn_conv_tc2_supported(const ConvGeom& g, const char** why);
 int mn_conv_tc2_launch(const ConvGeom& g, const void* w_hi, const void* w_lo, const float* w_scale, int prec, cudaStream_t st);
 // direct 3x3 conv for Cout <= 4 (conv_small.cu)

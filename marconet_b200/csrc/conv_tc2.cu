@@ -1,9 +1,17 @@
-// conv_tc2.cu -- second-generation tcgen05 operand-split implicit-GEMM convolution (see conv_tc.cu for the numerics:
-// x*w ~= xh*wh + (xh*wl + xl*wh), two fp32 TMEM accumulators, fp32 activations in HBM, A operand split on the fly into TMEM).
+// conv_tc2.cu -- tcgen05 / TMEM / TMA operand-split implicit-GEMM convolution for sm_100a: the tensor-core path of mn_conv2d_nhwc.
 //
-// v1 (conv_tc.cu) re-loads the 128-pixel activation tile once per tap and every CTA streams its own copy of the weights:
-// 64 KB of L2->SMEM traffic per 768 MMA cycles per SM, i.e. L2-bandwidth bound at ~36 % of the split-precision MMA peak.
-// v2 removes that traffic:
+// Numerics: the reference computes every conv in fp32 and the parity budget (1e-3 end to end, bit-exact argmax) rules out
+// single-pass fp16/bf16/tf32 operands (SURVEY.md section 0.7).  This kernel keeps fp32 activations in HBM and gets fp32-grade
+// products out of the fp16 tensor pipe by operand splitting:
+//     x = xh + xl,  w = wh + wl        (xh, xl, wh, wl fp16; |x - xh - xl| <= 2^-22 |x|)
+//     x*w ~= xh*wh + (xh*wl + xl*wh)   (three kind::f16 MMAs per k-step into two fp32 TMEM accumulators: D takes xh*wh, Dc the
+//                                       two cross terms; the epilogue adds D + Dc once, in fp32)
+// The tensor core truncates every add into an fp32 accumulator; with the cross terms (2^-11 of the result) kept apart, only K/16
+// instead of 3K/16 truncations hit the full-magnitude sum (DESIGN.md section 3.1).
+// The weights are split once by mn_conv_pack_weights_tc (end of this file), the activations on the fly by the split warps.
+//
+// Loading the 128-pixel activation tile once per tap, with every CTA streaming its own copy of the weights, would move 64 KB from
+// L2 to shared memory per 768 MMA cycles per SM and leave the kernel L2-bandwidth bound.  The design removes that traffic:
 //   * HALO TILE.  Loop order is (64-channel block) outer, (tap) inner.  One TMA box per channel block brings the
 //     (TH+2) x (TW+2) halo of the 128-pixel output tile (zero-filled outside the image = conv padding); the 9 taps are
 //     9 shifted *reads* of that tile by the split warps (row r of tap (ky,kx) is halo row r0 + ky*(TW+2) + kx).
@@ -677,6 +685,43 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
 }
 
+// ------------------------------------------------------------------------------------ weight packing
+__global__ void absmax_kernel(const float* __restrict__ w, int64_t n, float* __restrict__ out) {
+    float m = 0.f;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) m = fmaxf(m, fabsf(w[i]));
+    m = mn_warp_max(m);
+    if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int*>(out), __float_as_int(m));   // m >= 0: int order == float order
+}
+
+// w: [taps*Cin][Cout] fp32 (the SIMT layout) -> hi/lo 16-bit [taps][Cout][Cin] scaled by 2^S; scale[0] = absmax in,
+// scale[1] = 2^-S out.
+__global__ void pack_tc_kernel(const float* __restrict__ w, int taps, int Cin, int Cout, int bf, uint16_t* __restrict__ hi,
+                               uint16_t* __restrict__ lo, float* __restrict__ scale) {
+    const float amax = scale[0];
+    int e = 0;
+    if (amax > 0.f) { frexpf(amax, &e); }                 // amax = f * 2^e, f in [0.5,1)
+    const int S = bf ? 0 : (14 - e);                      // |w| * 2^S < 2^14
+    const float up = ldexpf(1.f, S);
+    if (blockIdx.x == 0 && threadIdx.x == 0) scale[1] = ldexpf(1.f, -S);
+    const int64_t total = (int64_t)taps * Cin * Cout;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int c = (int)(i % Cin);
+        const int64_t rest = i / Cin;
+        const int o = (int)(rest % Cout);
+        const int tap = (int)(rest / Cout);
+        const float v = w[((size_t)tap * Cin + c) * Cout + o] * up;
+        if (bf) {
+            const __nv_bfloat16 h = __float2bfloat16_rn(v);
+            const __nv_bfloat16 l = __float2bfloat16_rn(v - __bfloat162float(h));
+            hi[i] = *reinterpret_cast<const uint16_t*>(&h); lo[i] = *reinterpret_cast<const uint16_t*>(&l);
+        } else {
+            const __half h = __float2half_rn(v);
+            const __half l = __float2half_rn(v - __half2float(h));
+            hi[i] = *reinterpret_cast<const uint16_t*>(&h); lo[i] = *reinterpret_cast<const uint16_t*>(&l);
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------ host side
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -828,7 +873,7 @@ int mn_conv_tc2_supported(const ConvGeom& g, const char** why) {
 
 int mn_conv_tc2_launch(const ConvGeom& g, const void* w_hi, const void* w_lo, const float* w_scale, int prec, cudaStream_t st) {
     Tc2Plan p = plan_tc2(g);
-    if (!p.ok) { mn_set_error("mn_conv2d_nhwc: tcgen05 v2 path does not support this shape (%s)", p.why); return MN_ERR_UNSUPPORTED; }
+    if (!p.ok) { mn_set_error("mn_conv2d_nhwc: tensor-core path does not support this shape (%s)", p.why); return MN_ERR_UNSUPPORTED; }
     if (!w_hi || !w_lo || !w_scale) { mn_set_error("mn_conv2d_nhwc: tensor-core precision needs packed w_tc_hi/w_tc_lo/w_tc_scale"); return MN_ERR_INVALID; }
     PFN_encodeTiled enc = get_encode2();
     if (!enc) { mn_set_error("cuTensorMapEncodeTiled not available from the driver"); return MN_ERR_CUDA; }
@@ -870,4 +915,21 @@ int mn_conv_tc2_launch(const ConvGeom& g, const void* w_hi, const void* w_lo, co
     ConvGeom gr = g;
     gr.splits = t.ksplit;
     return mn_conv_splitk_reduce_launch(gr, st);
+}
+
+extern "C" int mn_conv_pack_weights_tc(const float* w, int taps, int Cin, int Cout, int precision, void* hi, void* lo,
+                                       float* scale2, void* stream) {
+    MN_REQUIRE(w && hi && lo && scale2 && taps > 0 && Cin > 0 && Cout > 0, "mn_conv_pack_weights_tc: bad args");
+    MN_REQUIRE(precision == MN_PREC_F16X3_TC || precision == MN_PREC_BF16X3_TC || precision == MN_PREC_F16X1_TC,
+               "mn_conv_pack_weights_tc: precision must be a tensor-core mode");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t total = (int64_t)taps * Cin * Cout;
+    MN_CUDA_CHECK(cudaMemsetAsync(scale2, 0, 2 * sizeof(float), st));
+    const int blocks = (int)(mn_cdiv64(total, 256) < 1184 ? mn_cdiv64(total, 256) : 1184);
+    absmax_kernel<<<blocks, 256, 0, st>>>(w, total, scale2);
+    MN_LAUNCH_CHECK();
+    pack_tc_kernel<<<blocks, 256, 0, st>>>(w, taps, Cin, Cout, precision == MN_PREC_BF16X3_TC ? 1 : 0,
+                                           reinterpret_cast<uint16_t*>(hi), reinterpret_cast<uint16_t*>(lo), scale2);
+    MN_LAUNCH_CHECK();
+    return MN_OK;
 }

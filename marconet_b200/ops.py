@@ -306,22 +306,12 @@ class calibration:
 TC_FALLBACKS = {}      # shape key -> (layer name, GFLOP, reason): convs that a tensor-core default ran on the fp32 CUDA-core kernel
 
 
-def _note_fallback(cw, key, flop, p):
+def _note_fallback(cw, key, flop, reason):
     """A tensor-core precision was the default but this conv runs on the exact fp32 kernel (unsupported geometry: Cin/Cout not
     multiples of 64, stride != 1, tiny launch ...).  Logged ONCE per shape so that a checkpoint with different channel counts does
     not quietly run 6x slower (VERDICT r1); ``ops.TC_FALLBACKS`` keeps the list, bench.py reports it."""
     if key in TC_FALLBACKS:
         return
-    if flop < TC_MIN_FLOP:
-        reason = f"below TC_MIN_FLOP ({flop / 1e6:.1f} MFLOP)"
-    elif cw is None or not cw.tc_capable():
-        reason = "Cin or Cout is not a multiple of 64"
-    elif key[7] != (1, 1):
-        reason = "stride != 1"
-    else:
-        lib = _lib.load()
-        lib.mn_conv2d_tc_supported(ctypes.byref(p))           # fills mn_last_error() with the kernel's own reason
-        reason = lib.mn_last_error().decode(errors="replace") or "unsupported geometry"
     name = cw.name if cw is not None else "unnamed"
     TC_FALLBACKS[key] = (name, flop / 1e9, reason)
     import logging
@@ -342,7 +332,7 @@ def conv2d(x, w, kh, kw, stride=(1, 1), pad=(0, 0), bias=None, out_scale=None, r
            res_broadcast=False, act=ACT_NONE, gain=1.0, out=None, out2=None, y2_scale=None,
            valid_w=None, precision=None, want_y=True, split_k=0, gn=None, gn_fuse=None, out2_ptrs=None, gn_stats=False):
     """mn_conv2d_nhwc.  ``w`` is the packed [KH*KW*Cin, Cout] matrix.  Returns y (or (y, y2)).
-    ``gn=(mean_rstd, gamma, beta)``: the conv input is swish(GroupNorm(x)); fused into the tcgen05 v2 kernel's operand-split
+    ``gn=(mean_rstd, gamma, beta)``: the conv input is swish(GroupNorm(x)); fused into the tcgen05 kernel's operand-split
     stage when ``gn_fuse`` is true and that kernel runs the layer, otherwise applied by mn_groupnorm_apply first.
     (Default on since the fused instantiation runs four lanes per halo row with the GroupNorm constants in registers: all eight
     normalise passes gone, 1.3 % per line on the same box, profiles/r2_split_gn_ab.txt; its first form -- one lane per row, per-row
@@ -402,12 +392,17 @@ def conv2d(x, w, kh, kw, stride=(1, 1), pad=(0, 0), bias=None, out_scale=None, r
     prec = precision if precision is not None else (cw.precision if (cw is not None and cw.precision is not None) else _DEFAULT_PRECISION)
     gn_fused = False
     if prec != PREC_FP32_SIMT:
-        ver = 0
-        if (cw is not None and cw.tc_capable() and stride == (1, 1)
-                and (precision is not None or 2.0 * n * oh * ow * cout * kh * kw * cin >= TC_MIN_FLOP)):
-            ver = lib.mn_conv2d_tc_version(ctypes.byref(p))
-        use_tc = ver > 0
-        if use_tc:
+        flop = 2.0 * n * oh * ow * cout * kh * kw * cin
+        why = None                            # why the tensor-core kernel does not run this conv
+        if precision is None and flop < TC_MIN_FLOP:
+            why = f"below TC_MIN_FLOP ({flop / 1e6:.1f} MFLOP)"
+        elif cw is None or not cw.tc_capable():
+            why = "Cin or Cout is not a multiple of 64"
+        elif stride != (1, 1):
+            why = "stride != 1"
+        elif not lib.mn_conv2d_tc_supported(ctypes.byref(p)):
+            why = lib.mn_last_error().decode(errors="replace") or "unsupported geometry"     # the kernel's planner says why
+        if why is None:
             hi, lo, sc = cw.tc(prec)
             p.w_tc_hi = hi.data_ptr(); p.w_tc_lo = lo.data_ptr(); p.w_tc_scale = sc.data_ptr()
             p.x_scale = cw.x_scale
@@ -415,18 +410,17 @@ def conv2d(x, w, kh, kw, stride=(1, 1), pad=(0, 0), bias=None, out_scale=None, r
             calib = getattr(_TLS, "calib", None)
             if calib is not None:
                 p.x_absmax = calib.slot(cw).data_ptr()
-            if gn is not None and ver == 2 and h * wd >= 128 and (_fuse_gn(cout) if gn_fuse is None else gn_fuse):   # one sample per 128-pixel tile
+            if gn is not None and h * wd >= 128 and (_fuse_gn(cout) if gn_fuse is None else gn_fuse):   # one sample per 128-pixel tile
                 p.gn_mean_rstd = gn[0].data_ptr(); p.gn_gamma = gn[1].data_ptr(); p.gn_beta = gn[2].data_ptr(); p.gn_swish = 1
                 gn_fused = True
         elif precision is not None:
-            raise RuntimeError("conv2d: tensor-core precision requested explicitly but this layer/shape is not supported: "
-                               + lib.mn_last_error().decode(errors="replace"))
+            raise RuntimeError("conv2d: tensor-core precision requested explicitly but this layer/shape is not supported: " + why)
         else:
             prec = PREC_FP32_SIMT
-            _note_fallback(cw, (n, h, wd, cin, cout, kh, kw, stride), 2.0 * n * oh * ow * cout * kh * kw * cin, p)
+            _note_fallback(cw, (n, h, wd, cin, cout, kh, kw, stride), flop, why)
     p.precision = prec
     stats_ws = None
-    if gn_stats and prec != PREC_FP32_SIMT and ver == 2 and oh * ow >= 128 and cout % 32 == 0 and y is not None and out2_ptrs is None:
+    if gn_stats and prec != PREC_FP32_SIMT and oh * ow >= 128 and cout % 32 == 0 and y is not None and out2_ptrs is None:
         stats_ws = torch.zeros((n * (cout // 32) * 2,), dtype=torch.float64, device=x.device)
         p.gn_stats_out = stats_ws.data_ptr()
     if gn is not None and not gn_fused:      # no fused kernel for this layer: normalise into a temporary first

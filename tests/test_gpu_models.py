@@ -29,7 +29,7 @@ TOL = 1e-3          # north_star budget (golden-fixture tests assert this)
 
 def _tol_internal():
     """Tighter bound the module-vs-oracle tests hold each path to: 2e-4 for the fp32 CUDA-core path, 5e-4 for the
-    tcgen05 operand-split path (its fp32 TMEM accumulation truncates; see conv_tc.cu)."""
+    tcgen05 operand-split path (its fp32 TMEM accumulation truncates; see conv_tc2.cu)."""
     from marconet_b200 import ops
     return 2e-4 if ops.default_precision() == ops.PREC_FP32_SIMT else 5e-4
 

@@ -135,8 +135,10 @@ def test_conv_tc_fused_groupnorm_swish(ragged, shape):
 
 
 def test_tc_unsupported_shape_is_reported():
+    """An explicit tensor-core precision on a 64->64 3x3 geometry the kernel's planner rejects raises, naming the planner's reason."""
     from marconet_b200 import ops
-    x = _rand(1, 64, 5, 7, seed=9)
     wt = _rand(64, 64, 3, 3, seed=10)
-    with pytest.raises(RuntimeError, match="not supported"):
-        ops.conv2d(_nhwc(x), _cw(wt), 3, 3, pad=(1, 1), precision=ops.PREC_F16X3_TC)
+    for h, w, reason in ((5, 7, "H must be a multiple of 8"), (12, 128, "H must be a multiple of 8"), (2, 256, "halo tile too large")):
+        x = _rand(1, 64, h, w, seed=9)
+        with pytest.raises(RuntimeError, match="not supported.*" + reason):
+            ops.conv2d(_nhwc(x), _cw(wt), 3, 3, pad=(1, 1), precision=ops.PREC_F16X3_TC)

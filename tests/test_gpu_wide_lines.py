@@ -131,9 +131,26 @@ def test_tspsrnet_rejects_what_the_reference_rejects_before_launching(gpu_models
             else:
                 sr.trunk(lq)
         assert ops.LAUNCHES == n0, shape
-    # H = 36 without characters is a valid reference call (no window is cut)
-    out = sr(torch.zeros((1, 3, 36, 512), device=dev), [p64[:0]], [p32[:0]], locs[:, :0])
-    assert out.shape == (1, 3, 144, 2048)
+    # H = 36 without characters is a valid reference call (no window is cut).  Its 36-, 18- and 9-row trunk layers are outside the
+    # tensor-core geometry: they run on the exact fp32 kernel, logged with the planner's reason, and the line matches the fp32 path.
+    lq36 = (torch.rand((1, 3, 36, 512), generator=torch.Generator().manual_seed(36)) * 2 - 1).to(dev)
+    saved, prec = dict(ops.TC_FALLBACKS), ops.default_precision()
+    try:
+        ops.TC_FALLBACKS.clear()
+        out = sr(lq36, [p64[:0]], [p32[:0]], locs[:, :0])
+        h_rows = {v[0]: k[1] for k, v in ops.TC_FALLBACKS.items() if "H must be a multiple of 8" in v[2]}
+        ops.set_default_precision(ops.PREC_FP32_SIMT)
+        ref = sr(lq36, [p64[:0]], [p32[:0]], locs[:, :0])
+    finally:
+        ops.set_default_precision(prec)
+        ops.TC_FALLBACKS.clear()
+        ops.TC_FALLBACKS.update(saved)
+    assert out.shape == ref.shape == (1, 3, 144, 2048)
+    assert h_rows == {"sr.conv_body_32.0": 36, "sr.conv_body_32.2": 36, "sr.conv_body_16.0": 18, "sr.conv_body_16.2": 18,
+                      "sr.conv_first_8.2": 9}, h_rows
+    err = float((out - ref).abs().max())
+    print("H = 36 line, tensor-core default vs fp32: max-abs", err)
+    assert err <= TOL
 
 
 def test_resample_modulate_checks_out_shape():
